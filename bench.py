@@ -6,6 +6,7 @@ multicommodity LP of configs[2] (both single-GPU profile workloads).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port of the reference PDLP on host cores
+  python bench.py ... --dump-outputs DIR                   # also save the last timed step's results as DIR/*.npy
 
 A "step" = one solve of ITERS_PER_STEP PDLP iterations on the resident LP (tolerances 0 => never stops early).
   value  = accepted PDLP iterations / device time of the solver loop (CUDA events, inputs resident in HBM)
@@ -222,6 +223,28 @@ def cusparse_comparator(lp, timeout_s=240):
     return None
 
 
+DUMP_SAMPLE = 1 << 21  # entries kept of a longer solution vector: 2 x 16 MB at float64
+
+
+def dump_outputs(out_dir, st, x, y):
+    """Writes one step's results as <out_dir>/<name>.npy so that two builds can be compared output for output.  A
+    vector longer than DUMP_SAMPLE is cut to the entries at the same seeded random positions on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def sample(v):
+        v = np.asarray(v, np.float64)
+        if v.size <= DUMP_SAMPLE:
+            return v
+        return v[np.sort(np.random.default_rng(0).choice(v.size, DUMP_SAMPLE, replace=False))]
+
+    arrays = {"primal_solution": sample(x), "dual_solution": sample(y)}
+    for name in ("primal_objective", "dual_objective", "relative_gap", "l2_relative_primal_residual",
+                 "l2_relative_dual_residual", "number_of_steps_taken"):
+        arrays[name] = np.array([getattr(st, name)], np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """CPU arm: the reference's PDLP as restated by the oracle port, all host threads, bounded sample."""
     rank = int(os.environ.get("RANK", "0"))
@@ -267,6 +290,10 @@ def main():
                     help="seconds given to the reference's own CPU path (dual simplex, 1 core) on this LP; 0 = skip")
     ap.add_argument("--comparator", default="auto", choices=["auto", "off"],
                     help="time the cuSPARSE/cuBLAS re-assembly of the reference's attempt (scripts/cusparse_pdhg.cu) beside ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to its caller as DIR/<name>.npy (float64): primal and "
+                         "dual solution (a fixed, seeded sample of DUMP_SAMPLE entries when longer), objectives, residuals "
+                         "and the iteration count; rank 0 only, so at N > 1 the dual is rank 0's block of rows")
     args = ap.parse_args()
     if args.cpu_iters <= 0:  # the OpenMP oracle runs roughly 1e8 nonzeros/s of PDHG iteration on 8 cores
         nnz_guess = {"c4": 80e6, "c2": 8e6, "c3": 0.9e6}[args.workload]
@@ -318,7 +345,7 @@ def main():
         x = sol.primal(); y = sol.dual()
         st = sol.stats()
         gsol_status[0] = sol.termination_reason
-        return st, float(x[0] + y[0])
+        return st, (x, y)
 
     def barrier():
         if world > 1:
@@ -334,7 +361,7 @@ def main():
     t0 = time.perf_counter()
     its = 0; dev_s = 0.0; launches = 0; setup_s = 0.0; loop_s = 0.0; term_s = 0.0
     for _ in range(args.steps):
-        st, _ = one_step()
+        st, last_xy = one_step()
         its += st.number_of_steps_taken
         dev_s += st.pdhg_loop_seconds + st.termination_seconds
         loop_s += st.pdhg_loop_seconds; term_s += st.termination_seconds
@@ -343,6 +370,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs and args.steps > 0:
+        dump_outputs(args.dump_outputs, st, *last_xy)
 
     # max over ranks (device time and wall), sum of iterations
     if world > 1:

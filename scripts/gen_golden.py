@@ -119,7 +119,34 @@ def main():
             value=32.0, abs=1e-3, source="cpp/tests/linear_programming/c_api_tests/c_api_test.c:761-874"),
     }
     json.dump(pins, open(os.path.join(GOLD, "reference_pins.json"), "w"), indent=1)
+    writer_golden()
+
+
+def writer_golden():
+    """writer_golden.json: the reference parser's reading of the MPS file this repo's writer writes for the LP of
+    tests/test_file_writers.py (needs cuopt_b200/lib/libcuopt.so too; the file is written before any GPU work)."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from cuopt_b200 import capi, lpgen
+    from test_file_writers import WRITER_LP, lp_digests, write_via_solve
+    lp = lpgen.sparse_lp(WRITER_LP["m"], WRITER_LP["n"], WRITER_LP["nnz_per_row"], seed=WRITER_LP["seed"])
+    p = capi.Problem.create_ranged(lp.offsets, lp.indices, lp.values, lp.con_lb, lp.con_ub, lp.c, lp.var_lb, lp.var_ub)
+    with tempfile.TemporaryDirectory() as tmp:
+        path = os.path.join(tmp, "written.mps")
+        write_via_solve(p, path)
+        m = ref_cpu.parse_mps(path)
+        with open(path, "rb") as f:
+            sha = hashlib.sha256(f.read()).hexdigest()
+    rec = dict(lp=f"lpgen.sparse_lp({WRITER_LP['m']}, {WRITER_LP['n']}, {WRITER_LP['nnz_per_row']}, "
+                  f"seed={WRITER_LP['seed']})", file_sha256=sha,
+               reference_parse=dict(m=m.m, n=m.n, digests=lp_digests(m.m, m.n, m.offsets, m.indices, m.values, m.c,
+                                                                     m.con_lb, m.con_ub, m.var_lb, m.var_ub)))
+    with open(os.path.join(GOLD, "writer_golden.json"), "w") as f:
+        json.dump(rec, f, indent=1)
+        f.write("\n")
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["writer"]:
+        writer_golden()
+    else:
+        main()

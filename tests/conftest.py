@@ -2,6 +2,7 @@ import gzip
 import json
 import os
 import sys
+import tempfile
 
 import numpy as np
 import pytest
@@ -19,14 +20,17 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "slow: larger sizes")
 
 
+_INFLATED = tempfile.TemporaryDirectory(prefix="cuopt_b200_mps_")  # removed when the session ends
+
+
 def mps_path(rel: str, tmp_dir=None) -> str:
-    """Path of a fixture under tests/golden/mps (gz files are inflated to a temp file)."""
+    """Path of a fixture under tests/golden/mps (gz files are inflated to a temp file: the tree may be read-only)."""
     p = os.path.join(MPS_DIR, rel)
     if os.path.exists(p):
         return p
     gz = p + ".gz"
     if os.path.exists(gz):
-        out_dir = tmp_dir or os.path.join(ROOT, "gpurun_out", "_tmp")
+        out_dir = tmp_dir or _INFLATED.name
         os.makedirs(out_dir, exist_ok=True)
         out = os.path.join(out_dir, os.path.basename(p))
         if not os.path.exists(out):

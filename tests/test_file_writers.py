@@ -1,12 +1,14 @@
 """`user_problem_file` / `solution_file` (constants.h parameter names; the reference's solve_lp writes them around the
 solve, cpp/src/linear_programming/solve.cu:586-601).  The MPS writer restates cpp/src/mip/problem/write_mps.cu; what it
-writes is read back by this repo's reader AND by the reference's own libmps_parser (oracle/_ref)."""
+writes is read back by this repo's reader AND, as recorded in tests/golden/writer_golden.json, by the reference's own
+libmps_parser."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
-from conftest import mps_path, problem_arrays
+from conftest import load_golden, mps_path, problem_arrays
 from cuopt_b200 import capi, lpgen
 
 
@@ -45,21 +47,33 @@ def test_written_mps_reads_back_identically(tmp_path, rel):
     assert a["maximize"] == b["maximize"] and p.is_mip == q.is_mip
 
 
-def test_reference_parser_reads_what_we_write(tmp_path):
-    from oracle import ref_cpu
-    if not ref_cpu.available():
-        pytest.skip("oracle/_ref not built")
-    lp = lpgen.sparse_lp(300, 250, 5, seed=3)   # E / L / G rows, x >= 0
-    p = capi.Problem.create_ranged(lp.offsets, lp.indices, lp.values, lp.con_lb, lp.con_ub, lp.c, lp.var_lb, lp.var_ub)
-    out = str(tmp_path / "written.mps")
-    write_via_solve(p, out)
-    m = ref_cpu.parse_mps(out)
+WRITER_LP = dict(m=300, n=250, nnz_per_row=5, seed=3)   # lpgen.sparse_lp: E / L / G rows, x >= 0
+
+
+def lp_digests(m, n, offsets, indices, values, c, con_lb, con_ub, var_lb, var_ub):
+    """Digests of an LP with its matrix in canonical CSR (a reader may order the entries of a row differently)."""
     import scipy.sparse as sp
-    A = sp.csr_matrix((lp.values, lp.indices, lp.offsets), shape=(lp.m, lp.n))
-    B = sp.csr_matrix((m.values, m.indices, m.offsets), shape=(lp.m, lp.n))
-    assert (A != B).nnz == 0
-    assert np.array_equal(m.c, lp.c) and np.array_equal(m.con_lb, lp.con_lb) and np.array_equal(m.con_ub, lp.con_ub)
-    assert np.array_equal(m.var_lb, lp.var_lb) and np.array_equal(m.var_ub, lp.var_ub)
+    A = sp.csr_matrix((np.asarray(values, np.float64), indices, offsets), shape=(m, n))
+    A.sort_indices()
+    arrays = dict(offsets=A.indptr.astype(np.int64), indices=A.indices.astype(np.int64), values=A.data, c=c,
+                  con_lb=con_lb, con_ub=con_ub, var_lb=var_lb, var_ub=var_ub)
+    return {k: hashlib.sha256(np.ascontiguousarray(a, dtype=np.int64 if k in ("offsets", "indices") else np.float64)
+                              .tobytes()).hexdigest()[:16] for k, a in arrays.items()}
+
+
+def test_reference_parser_reads_what_we_write(tmp_path):
+    # the reference's own libmps_parser read the file this writer writes for WRITER_LP back as exactly that LP
+    # (tests/golden/writer_golden.json, scripts/gen_golden.py); the verdict holds for a byte-identical file
+    gold = load_golden("writer_golden.json")
+    lp = lpgen.sparse_lp(WRITER_LP["m"], WRITER_LP["n"], WRITER_LP["nnz_per_row"], seed=WRITER_LP["seed"])
+    p = capi.Problem.create_ranged(lp.offsets, lp.indices, lp.values, lp.con_lb, lp.con_ub, lp.c, lp.var_lb, lp.var_ub)
+    out = tmp_path / "written.mps"
+    write_via_solve(p, str(out))
+    assert hashlib.sha256(out.read_bytes()).hexdigest() == gold["file_sha256"]
+    ref = gold["reference_parse"]
+    assert (ref["m"], ref["n"]) == (lp.m, lp.n)
+    assert ref["digests"] == lp_digests(lp.m, lp.n, lp.offsets, lp.indices, lp.values, lp.c, lp.con_lb, lp.con_ub,
+                                        lp.var_lb, lp.var_ub)
 
 
 def test_ranged_rows_are_written_like_the_reference_writes_them(tmp_path):

@@ -1,44 +1,39 @@
 """The two complete C programs of the reference's C-API documentation
-(docs/cuopt/source/cuopt-c/lp-milp/lp-example.rst: `lp_example.c`, `lp_example_mps.c`), extracted at build time,
-compiled UNCHANGED the way the documentation says (gcc -I include -L lib ... -lcuopt) against this repo's headers and
-library (oracle/Makefile target `ref`), and run here.  Expected values are the documentation's own "You should see
-the following output" blocks: Termination status: Optimal (1), Objective value: -0.360000, x1 = 1.800000,
-x2 = 0.000000.  (The solver's progress log differs: this build has no concurrent dual simplex to print about.)"""
-import os
-import re
-import subprocess
-
+(docs/cuopt/source/cuopt-c/lp-milp/lp-example.rst: `lp_example.c`, `lp_example_mps.c`), run against this repo's
+library through the same cuOpt* calls: the problem built from arrays, and the documentation's sample MPS file
+(tests/golden/mps/docs/lp_example_sample.mps).  Problem data and expected values are in tests/golden/c_api_problems.json;
+the values are the documentation's own "You should see the following output" blocks: Termination status: Optimal (1),
+Objective value: -0.360000, x1 = 1.800000, x2 = 0.000000."""
 import pytest
 
+from conftest import mps_path
+from cuopt_b200 import capi
+from test_reference_c_api_tests import SUCCESS, problem_data
+
 pytestmark = pytest.mark.gpu
-REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle", "_ref")
 
 
-def run(args):
-    exe = os.path.join(REF, args[0])
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref doc examples not built (needs /root/reference: make -C oracle ref)")
-    out = subprocess.run([exe] + args[1:], capture_output=True, text=True, timeout=300)
-    return out.returncode, out.stdout
-
-
-def check_results(text):
-    assert "Termination status: Optimal (1)" in text
-    obj = float(re.search(r"Objective value: (-?[0-9.]+)", text).group(1))
-    x1 = float(re.search(r"x1 = (-?[0-9.]+)", text).group(1))
-    x2 = float(re.search(r"x2 = (-?[0-9.]+)", text).group(1))
-    assert obj == pytest.approx(-0.36, abs=1e-4) and x1 == pytest.approx(1.8, abs=1e-3) and x2 == pytest.approx(0.0, abs=1e-3)
+def solve_like_the_example(p, d):
+    """cuOptCreateSolverSettings, absolute primal tolerance 1e-4, cuOptSolve, then what the example prints."""
+    s = capi.Settings()
+    assert capi.lib().cuOptSetFloatParameter(s.h, b"absolute_primal_tolerance", d["absolute_primal_tolerance"]) == SUCCESS
+    sol = capi.solve(p, s)
+    assert sol.return_code == SUCCESS, sol.error_string
+    assert sol.solve_time >= 0.0
+    assert sol.termination_status == d["expected_termination_status"]
+    assert sol.objective_value == pytest.approx(d["expected_objective"], abs=d["objective_abs"])
+    assert sol.primal() == pytest.approx(d["expected_primal"], abs=d["primal_abs"])
 
 
 def test_lp_example_with_data():
-    rc, text = run(["doc_lp_example"])
-    assert rc == 0, text
-    assert "Creating and solving simple LP problem..." in text and "Test completed successfully!" in text
-    check_results(text)
+    d = problem_data("doc_lp_example")
+    p = capi.Problem.create_ranged(d["offsets"], d["indices"], d["values"], d["con_lb"], d["con_ub"], d["c"],
+                                   d["var_lb"], d["var_ub"], maximize=d["maximize"],
+                                   variable_types=d["variable_types"].encode())
+    solve_like_the_example(p, d)
 
 
 def test_lp_example_with_mps_file():
-    rc, text = run(["doc_lp_example_mps", os.path.join(REF, "doc_sample.mps")])
-    assert rc == 0, text
-    assert "Number of variables: 2" in text and "Solver completed successfully!" in text
-    check_results(text)
+    p = capi.Problem.read(mps_path("docs/lp_example_sample.mps"))
+    assert p.num_variables == 2
+    solve_like_the_example(p, problem_data("doc_lp_example"))
